@@ -10,8 +10,10 @@
     parity    every run carries an in-run parity probe on the full-size data: chains {0, 1, C-1} stepped by the CPU oracle
               and by a `faithful` device handle, compared bit for bit; and a fast-vs-faithful two-sample KS
     --impl reference   the CPU restatement of mcmc.js (oracle/, Node is absent) on all host cores, one C call per step.
+    --dump-outputs DIR   after the timed steps, the draws of the last one as DIR/<name>.npy (see dump_outputs)
 
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0). Nothing is written into the source tree, which may be read-only: no bytecode, and the
+cubins of the run-time specialised sweep are cached in a temporary directory.
 """
 from __future__ import annotations
 
@@ -21,12 +23,14 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 import __graft_entry__ as graft  # noqa: E402
 
 METRIC = "posterior draws/sec (chains x iters) Normal(mu,sigma) N=1024 at 1/2/4/8 B200"
@@ -328,6 +332,26 @@ def parity_probe(cfg: Config, mcmc, orc, chains_total: int, device: int, seed: i
     return out
 
 
+DUMP_BYTES = 32 << 20          # --dump-outputs writes at most this many bytes of draws
+
+
+def dump_outputs(out_dir, sampler, cfg: Config, dev_out):
+    """--dump-outputs: what the last timed step returned, dev_out = [iters, entries, chains] float64 draws in HBM, written as
+    <name>.npy per parameter in the layout sample() returns ([iters, chains, *dim]). Above DUMP_BYTES a fixed seeded sample of the
+    chains is kept (and of the rows, if one chain's rows alone exceed it), so that runs with the same arguments compare file for file."""
+    import torch
+    rows, E, chains = dev_out.shape
+    rng = np.random.default_rng(0)
+    budget = DUMP_BYTES // 8
+    keep_rows = np.arange(rows) if rows * E <= budget else np.sort(rng.choice(rows, max(1, budget // E), replace=False))
+    keep_chains = np.sort(rng.choice(chains, min(chains, budget // (keep_rows.size * E)), replace=False))
+    sub = dev_out.index_select(0, torch.as_tensor(keep_rows, device=dev_out.device))
+    sub = sub.index_select(2, torch.as_tensor(keep_chains, device=dev_out.device)).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name in cfg.params:
+        np.save(os.path.join(out_dir, name + ".npy"), sampler._shape_out(name, sub[:, sampler._entries(name), :]))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -348,6 +372,11 @@ def run_ours(args):
     iters = args.iters or cfg.iters
     burn = cfg.burn if args.burn is None else args.burn
     seed = 0
+
+    jit_cache = None
+    if "AMWG_JIT_CACHE" not in os.environ:            # by default the library caches cubins next to itself, in the source tree
+        jit_cache = tempfile.TemporaryDirectory(prefix="amwg_jit_cache_")
+        os.environ["AMWG_JIT_CACHE"] = jit_cache.name
 
     chains_total = chains * world
     t_create = time.perf_counter()
@@ -410,6 +439,8 @@ def run_ours(args):
     dt = time.perf_counter() - t0
     launches = sampler.kernel_launches() - launches0
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sampler, cfg, dev_out)
     del dev_out
 
     # ---- the measured fp64 roof, same process, same clocks ------------------------------------------------------------
@@ -556,7 +587,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg and the parity probe")
     ap.add_argument("--no-probe", action="store_true", help="skip the in-run parity probe")
     ap.add_argument("--probe", action="store_true", help="force the in-run parity probe (default: single-GPU runs of configs 2-4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the draws of the last timed step as DIR/<name>.npy (float64; rank 0's chains, a fixed sample above 32 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU sampler (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,10 +1,12 @@
-"""bench.py, the parts that run without a GPU: the reference arm (`--impl reference`: the CPU restatement of mcmc.js on the host
-cores) prints ONE JSON line with the keys the driver's contract names, for the same metric / config / unit as the GPU arm; and the
-GPU arm refuses to run without a GPU instead of falling back to anything."""
+"""bench.py's command line. Without a GPU: the reference arm (`--impl reference`: the CPU restatement of mcmc.js on the host cores)
+prints ONE JSON line with the keys every bench line carries, for the same metric / config / unit as the GPU arm; the GPU arm refuses
+to run without a GPU instead of falling back to anything. On a GPU: --dump-outputs writes the draws of the last timed step."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -37,3 +39,36 @@ def test_gpu_arm_needs_a_gpu():
     r = _run(["--steps", "1", "--warmup", "3", "--no-cpu"], timeout=120)
     assert r.returncode != 0
     assert not [l for l in r.stdout.splitlines() if l.startswith("{")]      # no number without the CUDA path
+
+
+def test_bad_steps_and_dump_outputs_for_the_reference_arm_are_refused(tmp_path):
+    r = _run(["--steps", "0"], timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
+    r = _run(["--impl", "reference", "--dump-outputs", str(tmp_path / "out")], timeout=120)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "out").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_draws_of_the_last_timed_step(tmp_path, gpu_pkg):
+    """--dump-outputs writes what the last timed step drew: the arrays sample() returns for the same sweeps of the same chains, and
+    the same values again when bench.py runs a second time with the same arguments."""
+    import numpy as np
+    import models
+    from conftest import config2_data
+    args = ["--chains", "4096", "--iters", "10", "--burn", "20", "--steps", "2", "--warmup", "1", "--no-cpu"]
+    for run in ("a", "b"):
+        r = _run(args + ["--dump-outputs", str(tmp_path / run)], timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+        assert d["steps"] == 2 and d["warmup"] == 1
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("mu", "sigma")}
+    assert sorted(os.listdir(tmp_path / "a")) == ["mu.npy", "sigma.npy"]
+    for n, a in got.items():
+        assert a.dtype == np.float64 and a.shape == (10, 4096), (n, a.dtype, a.shape)
+        assert np.array_equal(a, np.load(tmp_path / "b" / f"{n}.npy")), n
+    s = gpu_pkg.mcmc.AmwgSampler(models.PARAMS_NORM, models.norm_post_readme(gpu_pkg.ld), config2_data().tolist(), {"chains": 4096, "seed": 0})
+    s.burn(20)
+    for _ in range(1 + 2):                              # warm-up + timed steps
+        want = s.sample(10)
+    for n, a in got.items():
+        assert np.array_equal(a, want[n]), n
