@@ -10,8 +10,11 @@
 // log_post(proposal) - log_post(current) as a sum of per-term differences instead of re-adding every cached term in order.
 #pragma once
 #include <dlfcn.h>
+#include <array>
 #include <map>
 #include <mutex>
+#include <regex>
+#include <set>
 #include <sstream>
 
 namespace jit {
@@ -566,6 +569,143 @@ static void emit_param_tables(std::ostringstream& tables, const amwg_model* md) 
 }
 
 
+// a run-time switch read when the specialisation is built (DESIGN.md section 6b): unset -> `dflt`, else its integer value != 0
+static bool env_flag(const char* name, bool dflt) {
+  const char* e = getenv(name);
+  return e ? atoi(e) != 0 : dflt;
+}
+
+struct StepClass { std::string body, commit; bool uses_m; };    // one `case` of jit_step as emit_step_class printed it
+
+// The merged form of jit_step (AMWG_JIT_MERGE_STEPS). The lanes of a warp step components of different classes at the same time
+// (each chain shuffles its substeppers), so in the switch form every class body -- with its out-of-line js_log / js_exp calls --
+// runs one after another under divergence. Here each class body is split into
+//   (A) per class: the operands of its heavy calls (a js_log / js_exp whose argument does not depend on another such call);
+//   (B) the heavy calls, once per warp: slot j of a function takes the j-th such call of every class (a class without one skips
+//       it behind a branch no lane of that class takes);
+//   (C) per class: the rest of the body in its original order -- every `dl = dl + ...` keeps its place, so dl is the same sum;
+//   one accept test for all classes; then the per-class commit.
+// Every value is computed by the same operations as in the switch form: the draws are bit-identical. Values cross the phases in
+// function-scope variables named k<class>_v<n>. false: the body text is not in the form emit_step_class prints.
+static bool emit_merged_step(const std::vector<StepClass>& cls, const std::string& accept_test, std::ostringstream& out) {
+  static const std::regex def_re("^    const double (v[0-9]+) = (.*);$"), name_re("\\bv[0-9]+\\b");
+  static const char* const kHeavy[2] = {"js_log", "js_exp"};
+  auto refs_of = [](const std::string& s) {
+    std::set<std::string> r;
+    for (std::sregex_iterator it(s.begin(), s.end(), name_re), e; it != e; ++it) r.insert(it->str());
+    return r;
+  };
+  auto heavy_of = [](const std::string& rhs, std::string& arg) -> int {     // rhs is exactly one call js_log(...) / js_exp(...)
+    for (int f = 0; f < 2; ++f) {
+      const std::string head = std::string(kHeavy[f]) + "(";
+      if (rhs.compare(0, head.size(), head) != 0 || rhs.back() != ')') continue;
+      int depth = 0;
+      for (size_t i = head.size() - 1; i < rhs.size(); ++i) {
+        depth += rhs[i] == '(' ? 1 : rhs[i] == ')' ? -1 : 0;
+        if (depth == 0 && i + 1 != rhs.size()) return -1;
+      }
+      arg = rhs.substr(head.size(), rhs.size() - head.size() - 1);
+      return f;
+    }
+    return -1;
+  };
+  struct Stmt { std::string text, name, rhs; bool def = false; int heavy = -1, slot = -1; std::string arg; bool phase_a = false; };
+  std::vector<std::vector<Stmt>> body(cls.size());
+  int n_slots[2] = {0, 0};
+  std::vector<std::array<std::vector<std::string>, 2>> args(cls.size());     // per class and function: the operand of each slot
+  bool uses_m = false;
+  for (size_t k = 0; k < cls.size(); ++k) {
+    uses_m = uses_m || cls[k].uses_m;
+    std::istringstream in(cls[k].body);
+    std::vector<Stmt>& st = body[k];
+    for (std::string ln; std::getline(in, ln);) {
+      Stmt s;
+      std::smatch mt;
+      if (ln.compare(0, 9, "    for (") == 0) {                 // a generated loop: one statement, to its closing brace
+        s.text = ln + "\n";
+        bool closed = false;
+        while (!closed && std::getline(in, ln)) { s.text += ln + "\n"; closed = ln == "    }"; }
+        if (!closed) return false;
+      } else if (std::regex_match(ln, mt, def_re)) {
+        s.def = true; s.name = mt[1]; s.rhs = mt[2];
+      } else {
+        s.text = ln + "\n";
+      }
+      st.push_back(s);
+    }
+    // heavy calls whose operand depends on no heavy result; `tainted`: every value that does
+    std::set<std::string> tainted;
+    int used[2] = {0, 0};
+    for (Stmt& s : st) {
+      if (!s.def) continue;
+      bool dep = false;
+      for (const auto& r : refs_of(s.rhs)) dep = dep || tainted.count(r);
+      std::string arg;
+      const int f = heavy_of(s.rhs, arg);
+      if (f >= 0 && !dep) { s.heavy = f; s.slot = used[f]++; s.arg = arg; args[k][f].push_back(arg); }
+      if (f >= 0 || dep) tainted.insert(s.name);
+    }
+    for (int f = 0; f < 2; ++f) n_slots[f] = std::max(n_slots[f], used[f]);
+    // (A) holds only what the operands need, so that little is live across the calls
+    std::set<std::string> need;
+    for (int f = 0; f < 2; ++f) for (const auto& a : args[k][f]) for (const auto& r : refs_of(a)) need.insert(r);
+    for (size_t i = st.size(); i-- > 0;)
+      if (st[i].def && st[i].heavy < 0 && need.count(st[i].name) && !tainted.count(st[i].name)) {
+        st[i].phase_a = true;
+        for (const auto& r : refs_of(st[i].rhs)) need.insert(r);
+      }
+  }
+  auto ren = [&](size_t k, const std::string& s) { return std::regex_replace(s, name_re, "k" + std::to_string(k) + "_$&"); };
+  auto slot_var = [](const char* pre, int f, int j) { return std::string(pre) + (f == 0 ? "l" : "e") + std::to_string(j); };
+  auto all_have = [&](int f, int j) { for (const auto& a : args) if ((int)a[f].size() <= j) return false; return true; };
+
+  out << "__device__ __forceinline__ bool jit_step(const int c, const double prop, const double coin, double* __restrict__ wk, const unsigned long long ws,\n"
+         "                                         double* __restrict__ sp, const unsigned long long ss) {\n";
+  if (uses_m) out << "  const int m = JMEM[c];\n";
+  for (size_t k = 0; k < cls.size(); ++k) {
+    std::string names;
+    for (const Stmt& s : body[k]) if (s.def) names += (names.empty() ? "" : ", ") + ren(k, s.name);
+    if (!names.empty()) out << "  double " << names << ";\n";
+  }
+  for (int f = 0; f < 2; ++f)
+    for (int j = 0; j < n_slots[f]; ++j) {
+      out << "  double " << slot_var("a", f, j) << " = 1.0;\n";
+      if (!all_have(f, j)) out << "  bool " << slot_var("u", f, j) << " = false;\n";
+    }
+  out << "  double dl = 0.0;\n  switch (JCLS[c]) {\n";              // (A)
+  for (size_t k = 0; k < cls.size(); ++k) {
+    out << "  case " << k << ": {\n";
+    for (const Stmt& s : body[k]) if (s.phase_a) out << "    " << ren(k, s.name) << " = " << ren(k, s.rhs) << ";\n";
+    for (int f = 0; f < 2; ++f)
+      for (int j = 0; j < (int)args[k][f].size(); ++j) {
+        out << "    " << slot_var("a", f, j) << " = " << ren(k, args[k][f][j]) << ";\n";
+        if (!all_have(f, j)) out << "    " << slot_var("u", f, j) << " = true;\n";
+      }
+    out << "    break;\n  }\n";
+  }
+  out << "  }\n";
+  for (int f = 0; f < 2; ++f)                                       // (B)
+    for (int j = 0; j < n_slots[f]; ++j) {
+      const std::string call = std::string(kHeavy[f]) + "(" + slot_var("a", f, j) + ")";
+      if (all_have(f, j)) out << "  const double " << slot_var("r", f, j) << " = " << call << ";\n";
+      else out << "  double " << slot_var("r", f, j) << " = 0.0;\n  if (" << slot_var("u", f, j) << ") " << slot_var("r", f, j) << " = " << call << ";\n";
+    }
+  out << "  switch (JCLS[c]) {\n";                                  // (C)
+  for (size_t k = 0; k < cls.size(); ++k) {
+    out << "  case " << k << ": {\n";
+    for (const Stmt& s : body[k]) {
+      if (s.phase_a) continue;
+      if (!s.def) out << ren(k, s.text);
+      else out << "    " << ren(k, s.name) << " = " << (s.heavy >= 0 ? slot_var("r", s.heavy, s.slot) : ren(k, s.rhs)) << ";\n";
+    }
+    out << "    break;\n  }\n";
+  }
+  out << "  }\n" << accept_test << "  ST(c) = prop;\n  switch (JCLS[c]) {\n";
+  for (size_t k = 0; k < cls.size(); ++k) out << "  case " << k << ": {\n" << ren(k, cls[k].commit) << "    break;\n  }\n";
+  out << "  }\n  return true;\n}\n";
+  return true;
+}
+
 // Build the specialised translation unit for `md`. Returns "" and fills `src` on success, else the reason it does not apply.
 static std::string build_source(const amwg_model* md, const std::vector<double>& consts, unsigned long long n_chains, int sm_count,
                                 double norm_c0, Source& src) {
@@ -673,6 +813,12 @@ static std::string build_source(const amwg_model* md, const std::vector<double>&
   }
   std::vector<int> cls_of(D, 0), mem_of(D, 0);
   funcs << "namespace amwg {\n";
+  const bool screen = env_flag("AMWG_JIT_ACCEPT_SCREEN", true);
+  const std::string accept_test = screen ? "    int acc_ = jit_accept_screen(dl, coin);              // certain from dl's sign or an fp32 estimate; -1: undecided\n"
+                                           "    if (acc_ < 0) acc_ = js_exp(dl) > coin;            // Metropolis accept (mcmc.js:527-534): strict >, NaN rejects\n"
+                                           "    if (!acc_) return false;\n"
+                                         : "    if (!(js_exp(dl) > coin)) return false;            // Metropolis accept (mcmc.js:527-534): strict >, NaN rejects\n";
+  std::vector<StepClass> step_classes;
   std::ostringstream step;
   step << "__device__ __forceinline__ bool jit_step(const int c, const double prop, const double coin, double* __restrict__ wk, const unsigned long long ws,\n"
           "                                         double* __restrict__ sp, const unsigned long long ss) {\n";
@@ -694,12 +840,17 @@ static std::string build_source(const amwg_model* md, const std::vector<double>&
     else step << "  {\n";
     if (inst.size() > 1) { step << "    const int m = JMEM[c];\n"; need_mem = true; }
     step << "    double dl = 0.0;\n" << body;
-    step << "    if (!(js_exp(dl) > coin)) return false;            // Metropolis accept (mcmc.js:527-534): strict >, NaN rejects\n";
+    step << accept_test;
     step << "    ST(c) = prop;\n" << commit;
     step << "    return true;\n  }\n";
+    step_classes.push_back(StepClass{body, commit, inst.size() > 1});
   }
   if (sig_order.size() > 1) step << "  }\n  return false;\n";
   step << "}\n";
+  if (sig_order.size() > 1 && env_flag("AMWG_JIT_MERGE_STEPS", true)) {
+    step.str("");
+    if (!emit_merged_step(step_classes, accept_test, step)) return "component program: unexpected generated step code";
+  }
 
   // ---- statistics whose mean is an expression
   std::ostringstream extra;

@@ -36,6 +36,29 @@ struct JitArgs {
 #define BC(c) wk[(unsigned long long)(2 * JNT + JD + (c)) * ws]
 #define ST(c) sp[(unsigned long long)(c) * ss]
 
+// The Metropolis decision js_exp(dl) > coin, taken without the fdlibm exp wherever it is certain (AMWG_JIT_ACCEPT_SCREEN).
+// 1 accept, 0 reject, -1 undecided: the caller then evaluates js_exp(dl) > coin itself. A lane that decides here skips the
+// out-of-line exp; a warp skips it when all its lanes do. coin is a uniform in [0, 1), and > 0 means >= 2^-53.
+//   * dl >= 0: js_exp(dl) >= 1 > coin (fdlibm returns 1 + dl below 2^-27 and is within 1 ulp of exp(dl) >= 1 + 2^-27 above).
+//   * dl < -40 (-inf too), coin > 0: js_exp(dl) <= exp(-40) (1 + 2^-52) < 4.3e-18 < 2^-53 <= coin.
+//   * -40 <= dl < 0: est = exp2f(t), t = (float)(dl * log2 e), |t| < 57.8. Relative error of est against exp(dl):
+//       the double product and the constant log2 e   <= 2^-51      (negligible: < 3e-14 absolute in t)
+//       rounding t to float (ulp <= 2^-18 below 64)  <= ln 2 * 2^-19 < 1.33e-6
+//       exp2f (CUDA: 2 ulp; glibc: 1 ulp), est >= 2^-58 is a normal float: <= 2^-22 < 2.4e-7
+//     so |est / exp(dl) - 1| < 1.6e-6, and js_exp(dl) is within 2^-52 of exp(dl). With the band B = 2^-16 (1.5e-5, nine times the
+//     error): est > coin (1 + B) proves exp(dl) > coin; est < coin (1 - B) proves js_exp(dl) <= coin. The products coin (1 +- B)
+//     round by 2^-53 relative, far inside the margin. A lane lands in the band with probability < 2 B.
+//   * NaN dl, coin == 0 and the band: undecided. (NaN compares false throughout; js_exp(NaN) > coin then rejects.)
+__device__ __forceinline__ int jit_accept_screen(const double dl, const double coin) {
+  if (dl >= 0.0) return 1;
+  if (!(coin > 0.0)) return -1;
+  if (dl < -40.0) return 0;
+  const double est = (double)exp2f((float)(dl * 1.4426950408889634));
+  if (est > coin * (1.0 + 0x1p-16)) return 1;
+  if (est < coin * (1.0 - 0x1p-16)) return 0;
+  return -1;
+}
+
 }  // namespace amwg
 
 #include "amwg_jit_generated.inc"
