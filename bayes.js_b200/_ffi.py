@@ -65,7 +65,7 @@ class AmwgModel(C.Structure):
 EXPORTS = ["amwg_create", "amwg_destroy", "amwg_burn", "amwg_sample", "amwg_sample_device", "amwg_get_state", "amwg_get_log_post",
            "amwg_set_adapting", "amwg_info", "amwg_kernel_launches", "amwg_last_sweep_kernel_ms", "amwg_n_chains",
            "amwg_last_error", "amwg_abi_version", "amwg_ld_eval", "amwg_primitive_eval",
-           "amwg_summary_moments", "amwg_summary_digit_hist", "amwg_peak_fp64", "amwg_jit_status", "amwg_jit_compile_check"]
+           "amwg_summary_moments", "amwg_summary_digit_hist", "amwg_summary_autocov", "amwg_peak_fp64", "amwg_jit_status", "amwg_jit_compile_check"]
 
 _lib = None
 
@@ -104,6 +104,7 @@ def lib():
     L.amwg_primitive_eval.argtypes = [i32, vp, i64, u64, u64, vp, C.c_int]; L.amwg_primitive_eval.restype = C.c_int
     L.amwg_summary_moments.argtypes = [C.c_int, vp, i64, i32, i64, vp]; L.amwg_summary_moments.restype = C.c_int
     L.amwg_summary_digit_hist.argtypes = [C.c_int, vp, i64, i32, i64, i32, vp, i32, vp]; L.amwg_summary_digit_hist.restype = C.c_int
+    L.amwg_summary_autocov.argtypes = [C.c_int, vp, i64, i32, i64, vp, vp, i32, i32, i32, vp]; L.amwg_summary_autocov.restype = C.c_int
     L.amwg_jit_status.argtypes = [vp, C.c_char_p, i64]; L.amwg_jit_status.restype = C.c_int
     L.amwg_jit_compile_check.argtypes = [C.POINTER(AmwgModel), u64, C.c_char_p, i64, C.c_char_p, i64]; L.amwg_jit_compile_check.restype = C.c_int
     L.amwg_peak_fp64.argtypes = [C.c_int, C.c_int, pd, pd]; L.amwg_peak_fp64.restype = C.c_int

@@ -543,15 +543,23 @@ class AmwgSampler(Sampler):
             raise JsThrow(L.amwg_last_error().decode())
         return buf
 
-    def sample_summary(self, n_iterations, probs=(0.025, 0.25, 0.5, 0.75, 0.975)):
+    def sample_summary(self, n_iterations, probs=(0.025, 0.25, 0.5, 0.75, 0.975), ess=False):
         """Not in the reference (SURVEY 8(f).3): the same sweeps and the same kept rows as `sample(n)` (thin / monitor apply), but the
         draws stay in HBM and only their summary comes back: {name: {"mean", "sd", "rhat", "quantiles", "n_draws"}}, pooled over
         all chains and kept rows; multi-dim parameters give arrays of their `dim` ("quantiles": [len(probs), *dim], exact order
         statistics with numpy.quantile's linear rule; a long grid such as numpy.linspace(0, 1, 41) gives an equal-mass histogram and
         runs as several radix selects of 16 probabilities each). With options.distributed every rank returns the all-GPU summary
-        (two small collectives, summary.py). Advances the chains exactly as sample(n) does."""
+        (two small collectives, summary.py). Advances the chains exactly as sample(n) does.
+
+        ess=True adds, per name and shaped like "mean": "ess", the bulk effective sample size of the mean on split chains without
+        rank normalisation (posterior::ess_mean, ArviZ ess(method="mean")); "ess_tail", the smaller ESS of the indicators x <= q05
+        and x <= q95 at the exact pooled 5 % / 95 % quantiles (posterior::ess_tail); "mcse", sd / sqrt(ess). NaN with fewer than 8
+        kept rows, for a constant entry or indicator, or when a draw is not finite. The autocovariances are reduced on the device
+        in tiles of lags, read only for the entries whose Geyer sequence is still positive (summary.summarise_ess). With
+        options.distributed every rank returns the same bits; they equal a single GPU's ESS to rounding, not bit for bit, because
+        the sums are grouped differently. The other fields are the same bits as with ess=False."""
         import torch
-        from .summary import CudaBlockReducer, summarise_block
+        from .summary import CudaBlockReducer, summarise_block, summarise_ess
         monitored = self._state_keys() if self.monitored_params is None else list(self.monitored_params)
         entries: List[int] = []
         spans = {}
@@ -580,11 +588,29 @@ class AmwgSampler(Sampler):
         if rc != 0:
             raise JsThrow(L.amwg_last_error().decode())
         t2 = time.perf_counter()
-        mean, sd, rhat, q = summarise_block(CudaBlockReducer(self.device), block, rows, self.n_chains, probs, self.distributed)
+        reducer = CudaBlockReducer(self.device)
+        if ess:                                                 # the tail ESS thresholds ride along in the same radix selects
+            probs = [float(p) for p in probs]
+            select = probs + [p for p in (0.05, 0.95) if p not in probs]
+            mean, sd, rhat, q = summarise_block(reducer, block, rows, self.n_chains, select, self.distributed)
+            t3 = time.perf_counter()
+            ess_v, tail_v, tiles = summarise_ess(reducer, block, rows, self.n_chains, q[select.index(0.05)], q[select.index(0.95)],
+                                                 self.distributed)
+            finite = np.isfinite(mean)                          # also covers the middle row of an odd `rows`, which no half-chain holds
+            ess_v, tail_v = np.where(finite, ess_v, np.nan), np.where(finite, tail_v, np.nan)
+            with np.errstate(invalid="ignore", divide="ignore"):
+                mcse = sd / np.sqrt(ess_v)
+            q = q[:len(probs)]
+        else:
+            mean, sd, rhat, q = summarise_block(reducer, block, rows, self.n_chains, probs, self.distributed)
         del block
         if timing:
+            t4 = time.perf_counter()
             print("sample_summary: alloc %.2f ms, sweeps %.2f ms, reductions %.2f ms" %
-                  (1e3 * (t1 - t0), 1e3 * (t2 - t1), 1e3 * (time.perf_counter() - t2)), file=sys.stderr, flush=True)
+                  (1e3 * (t1 - t0), 1e3 * (t2 - t1), 1e3 * (t4 - t2)), file=sys.stderr, flush=True)
+            if ess:
+                print("sample_summary: of which ess %.2f ms, %d lag tiles (mean, q05, q95 indicators; max per entry %d)" %
+                      (1e3 * (t4 - t3), int(tiles.sum()), int(tiles.max(initial=0))), file=sys.stderr, flush=True)
         out = {}
         for name in monitored:
             s0, ln = spans[name]
@@ -595,6 +621,8 @@ class AmwgSampler(Sampler):
             out[name] = {"mean": shape(mean[s0:s0 + ln]), "sd": shape(sd[s0:s0 + ln]), "rhat": shape(rhat[s0:s0 + ln]),
                          "quantiles": q[:, s0] if dim == [1] else q[:, s0:s0 + ln].reshape(len(q), *dim),
                          "n_draws": rows * self.n_chains}
+            if ess:
+                out[name].update(ess=shape(ess_v[s0:s0 + ln]), ess_tail=shape(tail_v[s0:s0 + ln]), mcse=shape(mcse[s0:s0 + ln]))
         return out
 
     def start_adaptation(self):

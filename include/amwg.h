@@ -272,10 +272,21 @@ AMWG_API int amwg_primitive_eval(int32_t kind, const double* x, int64_t n, uint6
  *   64-bit key of the draws: dev_counts[entry][prefix][256] += number of values of `entry` whose key's top 8*pass bits equal
  *   dev_prefix[entry][prefix] and whose next byte is the bin (pass 0 ignores the prefixes). Integer counts: exact and
  *   order-independent; the caller sums them over GPUs, picks the byte holding each wanted order statistic and extends the
- *   prefixes. n_prefix <= 32. */
+ *   prefixes. n_prefix <= 32.
+ *
+ * amwg_summary_autocov: split-chain autocovariance sums for the effective sample size. Per chain h = rows / 2; the half-chains are
+ *   the first and the last h rows (the middle row of an odd `rows` is dropped). y = x, or y = (x <= dev_threshold[entry] ? 1 : 0)
+ *   when dev_threshold (DEVICE, [entries]) is not NULL. For each live entry i (host_live[i], or every entry when host_live is
+ *   NULL) host_out[i][3 + n_lags] = { half-chains M', mean of the half-chain means, M2 of the half-chain means,
+ *   S_t for t = lag0 .. lag0 + n_lags - 1 }, S_t = sum over half-chains of sum_{n=0}^{h-1-t} (y_n - ybar)(y_{n+t} - ybar), ybar the
+ *   half-chain's mean (0 when t >= h). Merged in a fixed order (deterministic); a lag's sum has the same bits whatever lag0 and
+ *   n_lags. Shards merge like amwg_summary_moments records, with the S_t added. 8 <= rows < 2^31 - 64, 1 <= n_lags <= 16. */
 AMWG_API int amwg_summary_moments(int device, const double* dev_samples, int64_t rows, int32_t entries, int64_t chains, double* host_stats);
 AMWG_API int amwg_summary_digit_hist(int device, const double* dev_samples, int64_t rows, int32_t entries, int64_t chains, int32_t pass,
                                      const uint64_t* dev_prefix, int32_t n_prefix, uint64_t* dev_counts);
+AMWG_API int amwg_summary_autocov(int device, const double* dev_samples, int64_t rows, int32_t entries, int64_t chains,
+                                  const double* dev_threshold, const int32_t* host_live, int32_t n_live, int32_t lag0, int32_t n_lags,
+                                  double* host_out);
 
 /* ---- run-time specialisation ----------------------------------------------------------------------------------------------
  * For models that run the statistics sweep (stat_prog) amwg_create generates CUDA source from the model's programs, compiles it

@@ -355,6 +355,17 @@ BINDING(summary_digit_hist)
     fail_from_library();
   return js_undefined(env);
 END_BINDING
+// summary_autocov(device, samples ptr, rows, entries, chains, threshold ptr (0: none), lag0, n_lags) -> Float64Array [entries][3 + n_lags]
+//                                                                                 amwg_summary_autocov (every entry live)
+BINDING(summary_autocov)
+  const int32_t entries = (int32_t)to_double(env, a.at(3)), n_lags = (int32_t)to_double(env, a.at(7));
+  std::vector<double> out((size_t)std::max(entries, 0) * (size_t)(3 + std::max(n_lags, 0)));
+  if (amwg_summary_autocov((int)to_double(env, a.at(0)), (const double*)(uintptr_t)to_u64(env, a.at(1)), (int64_t)to_double(env, a.at(2)), entries,
+                           (int64_t)to_double(env, a.at(4)), (const double*)(uintptr_t)to_u64(env, a.at(5)), nullptr, 0, (int32_t)to_double(env, a.at(6)),
+                           n_lags, out.data()) != 0)
+    fail_from_library();
+  return f64_array(env, out.data(), out.size());
+END_BINDING
 // peak_fp64(device, reps) -> {tflops, ms}                                        amwg_peak_fp64
 BINDING(peak_fp64)
   double tf = 0.0, ms = 0.0;
@@ -393,7 +404,7 @@ NAPI_MODULE_INIT() {
       {"get_log_post", get_log_post}, {"set_adapting", set_adapting}, {"info", info}, {"kernel_launches", kernel_launches},
       {"last_sweep_kernel_ms", last_sweep_kernel_ms}, {"n_chains", n_chains}, {"last_error", last_error}, {"abi_version", abi_version},
       {"ld_eval", ld_eval}, {"primitive_eval", primitive_eval}, {"stream_uniforms", stream_uniforms}, {"device_log", device_log},
-      {"summary_moments", summary_moments}, {"summary_digit_hist", summary_digit_hist}, {"peak_fp64", peak_fp64}, {"jit_status", jit_status},
+      {"summary_moments", summary_moments}, {"summary_digit_hist", summary_digit_hist}, {"summary_autocov", summary_autocov}, {"peak_fp64", peak_fp64}, {"jit_status", jit_status},
       {"jit_compile_check", jit_compile_check}};
   for (const auto& e : table) {
     napi_value fn;
