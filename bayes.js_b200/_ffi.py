@@ -65,7 +65,8 @@ class AmwgModel(C.Structure):
 EXPORTS = ["amwg_create", "amwg_destroy", "amwg_burn", "amwg_sample", "amwg_sample_device", "amwg_get_state", "amwg_get_log_post",
            "amwg_set_adapting", "amwg_info", "amwg_kernel_launches", "amwg_last_sweep_kernel_ms", "amwg_n_chains",
            "amwg_last_error", "amwg_abi_version", "amwg_ld_eval", "amwg_primitive_eval",
-           "amwg_summary_moments", "amwg_summary_digit_hist", "amwg_summary_autocov", "amwg_peak_fp64", "amwg_jit_status", "amwg_jit_compile_check"]
+           "amwg_summary_moments", "amwg_summary_digit_hist", "amwg_summary_autocov", "amwg_summary_rank_keys", "amwg_summary_rank_sort",
+           "amwg_summary_rank_runs", "amwg_summary_rank_z", "amwg_summary_rank_scatter", "amwg_peak_fp64", "amwg_jit_status", "amwg_jit_compile_check"]
 
 _lib = None
 
@@ -105,6 +106,11 @@ def lib():
     L.amwg_summary_moments.argtypes = [C.c_int, vp, i64, i32, i64, vp]; L.amwg_summary_moments.restype = C.c_int
     L.amwg_summary_digit_hist.argtypes = [C.c_int, vp, i64, i32, i64, i32, vp, i32, vp]; L.amwg_summary_digit_hist.restype = C.c_int
     L.amwg_summary_autocov.argtypes = [C.c_int, vp, i64, i32, i64, vp, vp, i32, i32, i32, vp]; L.amwg_summary_autocov.restype = C.c_int
+    L.amwg_summary_rank_keys.argtypes = [C.c_int, vp, i64, i32, i64, i32, vp, vp, vp]; L.amwg_summary_rank_keys.restype = C.c_int
+    L.amwg_summary_rank_sort.argtypes = [C.c_int, vp, vp, i64, vp, vp, vp]; L.amwg_summary_rank_sort.restype = C.c_int
+    L.amwg_summary_rank_runs.argtypes = [C.c_int, vp, vp, vp, vp, i64, vp, vp, vp, vp]; L.amwg_summary_rank_runs.restype = C.c_int
+    L.amwg_summary_rank_z.argtypes = [C.c_int, vp, i64, i64, i64, vp]; L.amwg_summary_rank_z.restype = C.c_int
+    L.amwg_summary_rank_scatter.argtypes = [C.c_int, vp, vp, i64, vp, vp, i32, i64, i32]; L.amwg_summary_rank_scatter.restype = C.c_int
     L.amwg_jit_status.argtypes = [vp, C.c_char_p, i64]; L.amwg_jit_status.restype = C.c_int
     L.amwg_jit_compile_check.argtypes = [C.POINTER(AmwgModel), u64, C.c_char_p, i64, C.c_char_p, i64]; L.amwg_jit_compile_check.restype = C.c_int
     L.amwg_peak_fp64.argtypes = [C.c_int, C.c_int, pd, pd]; L.amwg_peak_fp64.restype = C.c_int

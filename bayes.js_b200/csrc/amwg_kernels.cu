@@ -1941,4 +1941,5 @@ extern "C" int amwg_primitive_eval(int32_t kind, const double* x, int64_t n, uin
 }
 
 #include "amwg_summary.cuh"
+#include "amwg_rank.cuh"
 #include "amwg_peak.cuh"

@@ -543,7 +543,7 @@ class AmwgSampler(Sampler):
             raise JsThrow(L.amwg_last_error().decode())
         return buf
 
-    def sample_summary(self, n_iterations, probs=(0.025, 0.25, 0.5, 0.75, 0.975), ess=False):
+    def sample_summary(self, n_iterations, probs=(0.025, 0.25, 0.5, 0.75, 0.975), ess=False, rank=False):
         """Not in the reference (SURVEY 8(f).3): the same sweeps and the same kept rows as `sample(n)` (thin / monitor apply), but the
         draws stay in HBM and only their summary comes back: {name: {"mean", "sd", "rhat", "quantiles", "n_draws"}}, pooled over
         all chains and kept rows; multi-dim parameters give arrays of their `dim` ("quantiles": [len(probs), *dim], exact order
@@ -557,9 +557,17 @@ class AmwgSampler(Sampler):
         kept rows, for a constant entry or indicator, or when a draw is not finite. The autocovariances are reduced on the device
         in tiles of lags, read only for the entries whose Geyer sequence is still positive (summary.summarise_ess). With
         options.distributed every rank returns the same bits; they equal a single GPU's ESS to rounding, not bit for bit, because
-        the sums are grouped differently. The other fields are the same bits as with ess=False."""
+        the sums are grouped differently. The other fields are the same bits as with ess=False.
+
+        rank=True (independent of ess) adds, per name and shaped like "mean", the rank-normalised diagnostics of Vehtari et al. (2021):
+        "rhat_bulk", the split R-hat of the rank-normalised split draws (ArviZ rhat(method="z_scale")); "rhat_folded", that of the
+        draws folded about their median; "rhat_rank", the larger of the two (posterior::rhat, ArviZ rhat(method="rank")); and
+        "ess_bulk", the Geyer ESS of the rank-normalised draws (posterior::ess_bulk). The exact pooled ranks come from a radix sort
+        on the device, entry by entry (summary.summarise_rank); with options.distributed the draws' runs are exchanged so that every
+        rank ranks over all chains, and every rank returns the same bits. NaN as for ess=True and when an entry is constant. The
+        other fields are the same bits as with rank=False."""
         import torch
-        from .summary import CudaBlockReducer, summarise_block, summarise_ess
+        from .summary import CudaBlockReducer, RankWorkingSetError, summarise_block, summarise_ess, summarise_rank
         monitored = self._state_keys() if self.monitored_params is None else list(self.monitored_params)
         entries: List[int] = []
         spans = {}
@@ -578,6 +586,21 @@ class AmwgSampler(Sampler):
         free, _total = torch.cuda.mem_get_info(dev)
         if need + 2 * len(entries) * self.local_chains * 8 > 0.9 * free:
             raise JsThrow("sample_summary: the sample block (%.1f GB) does not fit in device memory; raise thin() or lower n" % (need / 1e9))
+        h = rows // 2
+        if rank and h >= 4:
+            split = 2 * h * self.local_chains
+            if split >= 1 << 32:
+                raise JsThrow("sample_summary(rank=True): %d split draws of one entry on one GPU; the rank sort takes fewer than 2^32 "
+                              "(raise thin() or lower n)" % split)
+            # the z block, and per entry being sorted: keys and payloads double-buffered (24 B) and the sort's tile counts (1/4 B).
+            # Across GPUs the runs keep their keys (8 B) and each GPU merges the runs it receives (summary.RECV_BYTES_PER_RUN per
+            # run), counted here for as many runs as it sorted itself; the exchange checks the actual count again.
+            from .summary import RECV_BYTES_PER_RUN
+            per_draw = 24.25 + ((8 + RECV_BYTES_PER_RUN + 8) if self.distributed else 0)
+            need_rank = split * len(entries) * 8 + int(split * per_draw)
+            if need + need_rank + 2 * len(entries) * self.local_chains * 8 > 0.9 * free:
+                raise JsThrow("sample_summary(rank=True): the sample block (%.1f GB) and the rank working set (%.1f GB) do not fit in "
+                              "device memory; raise thin() or lower n" % (need / 1e9, need_rank / 1e9))
         timing = os.environ.get("AMWG_SUMMARY_TIMING") == "1"
         t0 = time.perf_counter()
         block = torch.empty((rows, len(entries), self.local_chains), dtype=torch.float64, device=dev)
@@ -589,10 +612,13 @@ class AmwgSampler(Sampler):
             raise JsThrow(L.amwg_last_error().decode())
         t2 = time.perf_counter()
         reducer = CudaBlockReducer(self.device)
+        M = rows * self.n_chains
+        middle = [M // 2 - 1, M // 2] if M % 2 == 0 else [M // 2]        # numpy.median's order statistics, for the fold
         if ess:                                                 # the tail ESS thresholds ride along in the same radix selects
             probs = [float(p) for p in probs]
             select = probs + [p for p in (0.05, 0.95) if p not in probs]
-            mean, sd, rhat, q = summarise_block(reducer, block, rows, self.n_chains, select, self.distributed)
+            res = summarise_block(reducer, block, rows, self.n_chains, select, self.distributed, middle if rank else ())
+            mean, sd, rhat, q = res[:4]
             t3 = time.perf_counter()
             ess_v, tail_v, tiles = summarise_ess(reducer, block, rows, self.n_chains, q[select.index(0.05)], q[select.index(0.95)],
                                                  self.distributed)
@@ -602,7 +628,20 @@ class AmwgSampler(Sampler):
                 mcse = sd / np.sqrt(ess_v)
             q = q[:len(probs)]
         else:
-            mean, sd, rhat, q = summarise_block(reducer, block, rows, self.n_chains, probs, self.distributed)
+            res = summarise_block(reducer, block, rows, self.n_chains, probs, self.distributed, middle if rank else ())
+            mean, sd, rhat, q = res[:4]
+        if rank:
+            t5 = time.perf_counter()
+            ost = res[4]
+            med = ost[0] if len(middle) == 1 else (ost[0] + ost[1]) / 2
+            rank_stats = {}
+            try:
+                r_bulk, r_fold, r_rank, ess_bulk = summarise_rank(reducer, block, rows, self.n_chains, med, self.distributed, rank_stats)
+            except RankWorkingSetError as e:
+                raise JsThrow(str(e)) from None
+            finite = np.isfinite(mean)
+            r_bulk, r_fold, r_rank, ess_bulk = (np.where(finite, a, np.nan) for a in (r_bulk, r_fold, r_rank, ess_bulk))
+            t6 = time.perf_counter()
         del block
         if timing:
             t4 = time.perf_counter()
@@ -610,7 +649,10 @@ class AmwgSampler(Sampler):
                   (1e3 * (t1 - t0), 1e3 * (t2 - t1), 1e3 * (t4 - t2)), file=sys.stderr, flush=True)
             if ess:
                 print("sample_summary: of which ess %.2f ms, %d lag tiles (mean, q05, q95 indicators; max per entry %d)" %
-                      (1e3 * (t4 - t3), int(tiles.sum()), int(tiles.max(initial=0))), file=sys.stderr, flush=True)
+                      (1e3 * (t5 - t3 if rank else t4 - t3), int(tiles.sum()), int(tiles.max(initial=0))), file=sys.stderr, flush=True)
+            if rank:
+                print("sample_summary: of which rank %.2f ms, %d sort passes run, %d skipped" %
+                      (1e3 * (t6 - t5), rank_stats.get("passes", 0), rank_stats.get("skipped", 0)), file=sys.stderr, flush=True)
         out = {}
         for name in monitored:
             s0, ln = spans[name]
@@ -623,6 +665,9 @@ class AmwgSampler(Sampler):
                          "n_draws": rows * self.n_chains}
             if ess:
                 out[name].update(ess=shape(ess_v[s0:s0 + ln]), ess_tail=shape(tail_v[s0:s0 + ln]), mcse=shape(mcse[s0:s0 + ln]))
+            if rank:
+                out[name].update(rhat_bulk=shape(r_bulk[s0:s0 + ln]), rhat_folded=shape(r_fold[s0:s0 + ln]),
+                                 rhat_rank=shape(r_rank[s0:s0 + ln]), ess_bulk=shape(ess_bulk[s0:s0 + ln]))
         return out
 
     def start_adaptation(self):

@@ -8,10 +8,12 @@ small collectives -- an all-gather of the per-rank moment records (merged exactl
 radix-select digit counts (integers) -- so every rank returns the same numbers as a single GPU holding all chains.
 
 With ess=True the summary also carries the effective sample size (`summarise_ess`): split-chain autocovariance sums over lag
-tiles, all-gathered and merged in rank order after each tile.
+tiles, all-gathered and merged in rank order after each tile. With rank=True it carries the rank-normalised split R-hat and bulk
+ESS (`summarise_rank`): exact pooled ranks from a device radix sort, the runs of equal values exchanged across GPUs.
 
 Host logic here is plain numpy (tested on CPU); the device work is behind `CudaBlockReducer` (C ABI: amwg_summary_moments,
-amwg_summary_digit_hist, amwg_summary_autocov). There is no CPU fallback: without the library or a GPU the reducer raises.
+amwg_summary_digit_hist, amwg_summary_autocov, amwg_summary_rank_*). There is no CPU fallback: without the library or a GPU the
+reducer raises.
 """
 from __future__ import annotations
 
@@ -179,10 +181,90 @@ class CudaBlockReducer:
                                                     int(lag0), int(n_lags), out.ctypes.data))
         return out
 
+    # ---- rank normalisation (include/amwg.h: amwg_summary_rank_*); the returned RankRuns keeps the device buffers alive
+    def rank_runs(self, block, entry: int, center, keep_keys: bool) -> "RankRuns":
+        """Sort the split draws of `entry` (folded about `center` unless None) and run-length encode them. keep_keys: also the
+        distinct keys (int64 view) and the sorted keys, for the exchange across GPUs."""
+        import torch
+        rows, entries, chains = block.shape
+        n = 2 * (rows // 2) * chains
+        dev = block.device
+        keys = torch.empty(n, dtype=torch.int64, device=dev)
+        vals = torch.empty(n, dtype=torch.int32, device=dev)
+        keys_alt = torch.empty_like(keys)
+        vals_alt = torch.empty_like(vals)
+        c = None if center is None else C.byref(C.c_double(float(center)))
+        torch.cuda.current_stream(dev).synchronize()
+        self._ffi.check(self.L.amwg_summary_rank_keys(self.device, block.data_ptr(), rows, entries, chains, int(entry), c,
+                                                      keys.data_ptr(), vals.data_ptr()))
+        passes = (C.c_int32 * 3)()
+        self._ffi.check(self.L.amwg_summary_rank_sort(self.device, keys.data_ptr(), vals.data_ptr(), n, keys_alt.data_ptr(),
+                                                      vals_alt.data_ptr(), passes))
+        if passes[2]:
+            keys, keys_alt, vals, vals_alt = keys_alt, keys, vals_alt, vals
+        # after the sort: vals_alt holds the run of each position, keys_alt the run counts; run keys only when asked for
+        runs = self._runs(keys, vals, None, vals_alt, keys_alt, torch.empty(n, dtype=torch.int64, device=dev) if keep_keys else None)
+        runs.passes, runs.skipped = int(passes[0]), int(passes[1])
+        runs.sorted_keys = keys
+        return runs
 
-def summarise_block(reducer, block, rows: int, total_chains: int, probs: Sequence[float], distributed: bool):
+    def _runs(self, keys, vals, weights, run_id, counts, run_keys) -> "RankRuns":
+        import torch
+        n = keys.numel()
+        n_runs = C.c_int64(0)
+        scan = None if weights is None else torch.empty(n, dtype=torch.int64, device=keys.device)
+        self._ffi.check(self.L.amwg_summary_rank_runs(self.device, keys.data_ptr(), vals.data_ptr(),
+                                                      None if weights is None else weights.data_ptr(),
+                                                      None if scan is None else scan.data_ptr(), n, run_id.data_ptr(),
+                                                      None if run_keys is None else run_keys.data_ptr(), counts.data_ptr(), C.byref(n_runs)))
+        r = n_runs.value
+        return RankRuns(vals, run_id, counts[:r], None if run_keys is None else run_keys[:r], n)
+
+    def rank_merge(self, keys, counts) -> "RankRuns":
+        """Owner side across GPUs: the received (key, count) pairs sorted by key (payload: the receive index), equal keys'
+        counts summed. `keys` (int64 view) is sorted in place: the caller gives up its contents. Device memory while it runs:
+        40 B per received pair with `keys` and `counts`; 16 B per pair stay in the result."""
+        import torch
+        n = keys.numel()
+        dev = keys.device
+        if n == 0:
+            e = torch.empty(0, dtype=torch.int64, device=dev)
+            return RankRuns(torch.empty(0, dtype=torch.int32, device=dev), torch.empty(0, dtype=torch.int32, device=dev), e, e, 0)
+        k = keys
+        v = torch.arange(n, dtype=torch.int32, device=dev)
+        k_alt, v_alt = torch.empty_like(k), torch.empty_like(v)
+        passes = (C.c_int32 * 3)()
+        torch.cuda.current_stream(dev).synchronize()
+        self._ffi.check(self.L.amwg_summary_rank_sort(self.device, k.data_ptr(), v.data_ptr(), n, k_alt.data_ptr(), v_alt.data_ptr(), passes))
+        if passes[2]:
+            k, k_alt, v, v_alt = k_alt, k, v_alt, v
+        return self._runs(k, v, counts.contiguous(), v_alt, k_alt, None)
+
+    def rank_z(self, counts, offset: int, total: int, out=None):
+        """-> float64 tensor (`out` when given): z per run (include/amwg.h amwg_summary_rank_z)."""
+        import torch
+        z = torch.empty(counts.numel(), dtype=torch.float64, device=counts.device) if out is None else out
+        if counts.numel():
+            torch.cuda.current_stream(counts.device).synchronize()
+            self._ffi.check(self.L.amwg_summary_rank_z(self.device, counts.data_ptr(), counts.numel(), int(offset), int(total), z.data_ptr()))
+        return z
+
+    def rank_scatter(self, runs: "RankRuns", run_z, out, entry: int) -> None:
+        """out[2h, entries, chains]: the z of every split draw of `entry`; out 1-d: out[payload] (the owner's reply)."""
+        import torch
+        if runs.n == 0:
+            return
+        torch.cuda.current_stream(out.device).synchronize()
+        entries, chains = (out.shape[1], out.shape[2]) if out.dim() == 3 else (1, out.numel())
+        self._ffi.check(self.L.amwg_summary_rank_scatter(self.device, runs.vals.data_ptr(), runs.run_id.data_ptr(), runs.n,
+                                                         run_z.data_ptr(), out.data_ptr(), entries, chains, int(entry)))
+
+
+def summarise_block(reducer, block, rows: int, total_chains: int, probs: Sequence[float], distributed: bool, order_stats: Sequence[int] = ()):
     """-> (mean, sd, rhat, quantiles[len(probs)]) per entry, over all shards. `reducer` does the per-shard device work;
-    the collectives run on the tensors it returns (NCCL for CUDA tensors, gloo for the CPU stand-in used in the tests)."""
+    the collectives run on the tensors it returns (NCCL for CUDA tensors, gloo for the CPU stand-in used in the tests).
+    With order_stats (0-based ranks over all rows * total_chains draws) also -> [len(order_stats), entries] those order
+    statistics, selected in the first radix select alongside the quantiles (the quantiles are the same bits either way)."""
     import torch
     entries = block.shape[1]
     rec = reducer.moments(block)
@@ -199,10 +281,22 @@ def summarise_block(reducer, block, rows: int, total_chains: int, probs: Sequenc
 
     probs = [float(p) for p in probs]
     q = np.empty((len(probs), entries))
+    extra = np.asarray(order_stats, dtype=np.int64)
+    ostat = np.empty((len(extra), entries))
     per_select = MAX_PREFIXES // 2                            # every probability needs at most two order statistics
-    for first in range(0, len(probs), per_select):            # long probability grids (equal-mass histograms): several selects
-        chunk = probs[first:first + per_select]
+    chunks, first = [], 0
+    while first < len(probs) or (len(extra) and not chunks):  # long probability grids (equal-mass histograms): several selects
+        size = per_select - ((len(extra) + 1) // 2 if not chunks else 0)
+        chunks.append(first)
+        first += size
+    for ci, first in enumerate(chunks):
+        chunk = probs[first:chunks[ci + 1] if ci + 1 < len(chunks) else len(probs)]
         ranks, plan = quantile_targets(rows * total_chains, chunk)
+        if ci == 0 and len(extra):
+            union = np.union1d(ranks, extra)
+            pos = np.searchsorted(union, ranks)
+            plan = [(pos[lo], pos[hi], g) for lo, hi, g in plan]
+            ranks = union
         sel = RadixSelect(entries, ranks)
         for npass in range(8):
             table, which = sel.prefixes()
@@ -214,6 +308,10 @@ def summarise_block(reducer, block, rows: int, total_chains: int, probs: Sequenc
         vals = sel.values()                                   # [entries, T]
         for i, (lo, hi, g) in enumerate(plan):
             q[first + i] = _lerp(vals[:, lo], vals[:, hi], g)
+        if ci == 0 and len(extra):
+            ostat[:] = vals[:, np.searchsorted(ranks, extra)].T
+    if len(extra):
+        return mean, sd, rhat, q, ostat
     return mean, sd, rhat, q
 
 
@@ -289,9 +387,10 @@ def _gather_autocov(out: np.ndarray, block) -> np.ndarray:
     return np.concatenate([rec[:, :3], s], axis=1)
 
 
-def _ess_pass(reducer, block, h: int, thresholds, distributed: bool):
+def _ess_pass(reducer, block, h: int, thresholds, distributed: bool, want_record: bool = False):
     """-> (ess [entries], lag tiles read per entry). Every entry starts live; after each tile of reducer.lag_tile lags the entries
-    whose sequence has ended drop out, and only the live ones are read for the next tile."""
+    whose sequence has ended drop out, and only the live ones are read for the next tile. want_record: also -> the first tile's
+    [entries, 4] (half-chains, mean and M2 of the half-chain means, S_0), merged over all shards."""
     entries = block.shape[1]
     L = reducer.lag_tile
     ess = np.full(entries, np.nan)
@@ -305,7 +404,7 @@ def _ess_pass(reducer, block, h: int, thresholds, distributed: bool):
         if distributed:
             out = _gather_autocov(out, block)
         if rec is None:
-            rec = out[:, :3].copy()                  # the first tile covers every entry
+            rec = out[:, :4].copy()                  # the first tile covers every entry
         nxt = []
         for i, e in enumerate(live):
             S[e] = np.concatenate([S[e], out[i, 3:]])
@@ -317,6 +416,8 @@ def _ess_pass(reducer, block, h: int, thresholds, distributed: bool):
                 ess[e] = r
         live = np.asarray(nxt, dtype=np.int64)
         lag0 += L
+    if want_record:
+        return ess, tiles, rec
     return ess, tiles
 
 
@@ -335,3 +436,169 @@ def summarise_ess(reducer, block, rows: int, total_chains: int, q05, q95, distri
     e95, t2 = _ess_pass(reducer, block, h, np.asarray(q95, dtype=np.float64), distributed)
     tail = np.where(np.isnan(ess), np.nan, np.minimum(e05, e95))      # a non-finite draw leaves the indicators finite
     return ess, tail, np.stack([t0, t1, t2])
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# rank-normalised split R-hat and bulk ESS (Vehtari, Gelman, Simpson, Carpenter, Buerkner 2021; posterior::rhat, ess_bulk)
+#
+# Split: per chain h = rows // 2, the half-chains are the first h and the last h kept rows (the middle row of an odd `rows` is
+# dropped, as posterior split_chains / ArviZ _split_chains); S = 2h x total chains split draws per entry.
+# Ranks: average ranks (ties get the mean of their positions, scipy.stats.rankdata(method="average")) of the S split draws of the
+# entry, pooled over all chains on all GPUs; -0.0 and +0.0 tie. z = Phi^-1((r - 3/8) / (S + 1/4)) (CUDA normcdfinv on the device).
+# Fold: zeta = |x - med|, med = numpy.median of all rows x chains draws (the middle row included), (a + b) / 2 of the two middle
+# order statistics; zeta goes through the same split, rank and z steps.
+# Split R-hat of a z block from the first tile of amwg_summary_autocov (M' half-chains, M2 of the half-chain means, S_0):
+#   W = S_0 / (M'(h-1)),   var+ = (h-1)/h W + M2_means / (M'-1),   R-hat = sqrt(var+ / W)
+# rhat_bulk is that of z, rhat_folded that of the folded z, rhat_rank = max(rhat_bulk, rhat_folded); ess_bulk is geyer_ess of z
+# (the loop bounds above). NaN with fewer than 8 kept rows, when a split draw is not finite, and when W or var+ is 0 (a constant
+# entry ties everywhere: z = 0).
+#
+# Several GPUs: the ranks must be exact over all shards. Every rank sorts its own draws and run-length encodes them into
+# (key, count) runs. Regular-sampling splitters: each rank contributes G keys at evenly spaced positions of its sorted draws, they
+# are all-gathered and sorted, and every G-th one is a splitter. A run goes to the owner of its key's range (key < splitter), so all
+# copies of a value meet at one owner; all_to_all_single moves the runs (keys as an int64 view), the owner merges them (the same
+# sort, counts of equal keys summed), its rank offset is the scan of the owners' totals (one all-gather of one integer), and the z
+# of every run returns by the reverse all_to_all_single. So every rank's z block is the matching slice of a single GPU's, bit for bit.
+class RankRuns:
+    """One sorted, run-length encoded key set: vals (payload per sorted position), run_id (run per sorted position), counts (per
+    run), keys (per run, int64 view, or None), n (keys sorted)."""
+
+    def __init__(self, vals, run_id, counts, keys, n: int):
+        self.vals, self.run_id, self.counts, self.keys, self.n = vals, run_id, counts, keys, n
+        self.passes = self.skipped = 0
+        self.sorted_keys = None
+
+
+_KEY_FLIP = -(1 << 63)                 # x ^ _KEY_FLIP on an int64 view: signed order == the keys' unsigned order
+RECV_BYTES_PER_RUN = 40 + 16           # the owner's merge (rank_merge with the received keys and counts), then z owned + z sent back
+
+
+class RankWorkingSetError(MemoryError):
+    """The runs one GPU receives in the exchange do not fit in its free device memory (raised on every rank alike)."""
+
+
+def _device_free(dev) -> int:
+    """bytes a new tensor can take: free device memory plus what torch's allocator holds unused"""
+    import torch
+    free, _ = torch.cuda.mem_get_info(dev)
+    return free + torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev)
+
+
+def _exchange_z(reducer, runs: RankRuns, total: int):
+    """-> float64 tensor [runs]: the z of this rank's runs, ranked over all ranks' draws (above). Before the runs move, every rank
+    checks that what it will receive fits (RECV_BYTES_PER_RUN per received run); when one does not, all raise RankWorkingSetError."""
+    import torch
+    import torch.distributed as dist
+    G, me = dist.get_world_size(), dist.get_rank()
+    dev = runs.counts.device
+    n_runs = runs.counts.numel()
+    pos = torch.tensor([(i * runs.n) // G for i in range(G)], dtype=torch.int64, device=dev)
+    samples = runs.sorted_keys[pos].contiguous()
+    runs.sorted_keys = None                                   # spent: its memory goes to the receive side
+    every = torch.empty(G * G, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(every, samples)
+    u = np.sort(every.cpu().numpy().view(np.uint64))
+    splitters = u[G::G][:G - 1]
+    flipped = lambda k: k ^ _KEY_FLIP
+    cut = torch.searchsorted(flipped(runs.keys), flipped(torch.from_numpy(splitters.view(np.int64).copy()).to(dev))) if G > 1 else \
+        torch.empty(0, dtype=torch.int64, device=dev)
+    bounds = [0] + cut.cpu().tolist() + [n_runs]
+    send = [bounds[j + 1] - bounds[j] for j in range(G)]
+    sizes = torch.tensor(send, dtype=torch.int64, device=dev)
+    got = torch.empty_like(sizes)
+    dist.all_to_all_single(got, sizes)
+    recv = got.cpu().tolist()
+    R = sum(recv)
+    short = torch.zeros(1, dtype=torch.int64, device=dev)
+    need = RECV_BYTES_PER_RUN * R + R // 4 + 8 * n_runs         # + the sort's tile counts, + this rank's z
+    if dev.type == "cuda" and need > 0.9 * _device_free(dev):
+        short[0] = need
+    dist.all_reduce(short, op=dist.ReduceOp.MAX)
+    if int(short.item()):
+        raise RankWorkingSetError("sample_summary(rank=True): a GPU would receive runs needing %.1f GB in the exchange of ranks, "
+                                  "more than its free device memory; raise thin() or lower n" % (int(short.item()) / 1e9))
+    keys_in = torch.empty(R, dtype=torch.int64, device=dev)
+    counts_in = torch.empty(R, dtype=torch.int64, device=dev)
+    dist.all_to_all_single(keys_in, runs.keys.contiguous(), recv, send)
+    dist.all_to_all_single(counts_in, runs.counts.contiguous(), recv, send)
+    owned = reducer.rank_merge(keys_in, counts_in)              # sorts keys_in in place
+    del keys_in
+    mine = counts_in.sum().reshape(1).to(torch.int64)
+    del counts_in
+    totals = torch.empty(G, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(totals, mine)
+    offset = int(totals[:me].sum().item())
+    z_owned = reducer.rank_z(owned.counts, offset, total)
+    z_in = torch.empty(R, dtype=torch.float64, device=dev)
+    reducer.rank_scatter(owned, z_owned, z_in, 0)
+    del owned, z_owned
+    z = torch.empty(n_runs, dtype=torch.float64, device=dev)
+    dist.all_to_all_single(z, z_in, send, recv)
+    return z
+
+
+def rank_normalise(reducer, block, rows: int, total_chains: int, center, distributed: bool, out=None, stats=None):
+    """-> (z block [2h, entries, chains] (float64, on the block's device; `out` when given), finite [entries] bool): the
+    rank-normalised split draws of every entry (definition above), folded about center[entry] unless center is None. Entries go
+    through the sort one at a time. finite: every split draw of the entry is finite, over all shards. stats (a dict) collects the
+    sort passes run and skipped."""
+    import torch
+    h = rows // 2
+    _, entries, chains = block.shape
+    if out is None:
+        out = torch.empty((2 * h, entries, chains), dtype=torch.float64, device=block.device)
+    total = 2 * h * total_chains
+    lo_inf, hi_inf = double_to_key(np.array([-np.inf, np.inf]))
+    finite = np.ones(entries, dtype=np.int64)
+    for e in range(entries):
+        runs = reducer.rank_runs(block, e, None if center is None else float(center[e]), distributed)
+        if stats is not None:
+            stats["passes"] = stats.get("passes", 0) + runs.passes
+            stats["skipped"] = stats.get("skipped", 0) + runs.skipped
+        ends = runs.sorted_keys[[0, -1]].cpu().numpy().view(np.uint64)
+        if distributed:
+            z = _exchange_z(reducer, runs, total)
+        else:                                                  # the sorted keys are spent: their buffer takes the z
+            z = reducer.rank_z(runs.counts, 0, total, out=runs.sorted_keys.view(torch.float64)[:runs.counts.numel()])
+        finite[e] = int(ends[0] > lo_inf and ends[1] < hi_inf)
+        reducer.rank_scatter(runs, z, out, e)
+        del runs, z
+    if distributed:
+        import torch.distributed as dist
+        f = torch.from_numpy(finite).to(block.device)
+        dist.all_reduce(f, op=dist.ReduceOp.MIN)
+        finite = f.cpu().numpy()
+    return out, finite.astype(bool)
+
+
+def split_rhat(rec: np.ndarray, h: int) -> np.ndarray:
+    """R-hat per entry from [entries, >= 4] (half-chains M', mean and M2 of the half-chain means, S_0) of amwg_summary_autocov."""
+    M, m2, S0 = rec[:, 0], rec[:, 2], rec[:, 3]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        W = S0 / (M * (h - 1))
+        var_plus = (h - 1) / h * W + m2 / (M - 1)
+        ok = (W > 0) & (var_plus > 0) & np.isfinite(W) & np.isfinite(var_plus)
+        return np.where(ok, np.sqrt(np.where(ok, var_plus / W, 1.0)), np.nan)
+
+
+def summarise_rank(reducer, block, rows: int, total_chains: int, med, distributed: bool, stats=None):
+    """-> (rhat_bulk, rhat_folded, rhat_rank, ess_bulk) per entry over all shards (definition above). med: numpy.median of
+    every draw of each entry. One z block: the bulk z for ess_bulk and rhat_bulk (the first lag tile's record, merged over the
+    shards), then refilled with the folded z for one single-lag autocovariance call. Every rank returns the same bits."""
+    entries = block.shape[1]
+    h = rows // 2
+    nan = np.full(entries, np.nan)
+    if h < 4:
+        return nan, nan.copy(), nan.copy(), nan.copy()
+    z, finite = rank_normalise(reducer, block, rows, total_chains, None, distributed, stats=stats)
+    ess, _, rec = _ess_pass(reducer, z, h, None, distributed, want_record=True)
+    bulk = split_rhat(rec, h)
+    z, finite_f = rank_normalise(reducer, block, rows, total_chains, med, distributed, out=z, stats=stats)
+    out = reducer.autocov(z, None, np.arange(entries), 0, 1)
+    if distributed:
+        out = _gather_autocov(out, z)
+    folded = split_rhat(out, h)
+    del z
+    ok = finite & finite_f
+    bulk, folded = np.where(ok, bulk, np.nan), np.where(ok, folded, np.nan)
+    return bulk, folded, np.maximum(bulk, folded), np.where(ok, ess, np.nan)

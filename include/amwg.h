@@ -288,6 +288,40 @@ AMWG_API int amwg_summary_autocov(int device, const double* dev_samples, int64_t
                                   const double* dev_threshold, const int32_t* host_live, int32_t n_live, int32_t lag0, int32_t n_lags,
                                   double* host_out);
 
+/* ---- rank normalisation (sample_summary(rank=True)) ------------------------------------------------------------------------
+ * The exact pooled average rank of every split draw of one entry, and z = Phi^-1((r - 3/8) / (S + 1/4)) (Vehtari et al. 2021),
+ * in five steps that the caller chains (and, across GPUs, interleaves with an exchange of the runs: summary.py). All pointers
+ * named dev_ are DEVICE memory owned by the caller; keys are the order-preserving 64-bit keys of amwg_summary_digit_hist, with
+ * -0 canonicalised to +0 (so -0 and +0 tie). n (keys, draws) must be 1 <= n < 2^32; the library's own scratch is about
+ * n / 4 bytes during a sort, released when the call ends (only scratch up to 64 MiB is kept between calls). Every call returns
+ * after its work is complete.
+ *
+ * amwg_summary_rank_keys: the split draws of `entry` (per chain h = rows / 2: the first and the last h rows; the middle row of an
+ *   odd `rows` is dropped), S = 2h * chains of them, folded to |x - *host_center| when host_center is not NULL ->
+ *   dev_keys[S] and dev_vals[S] = r' * chains + c, the position in a split block [2h][chains] (r' = 0 .. 2h - 1).
+ * amwg_summary_rank_sort: stable LSD radix sort of the (key, u32) pairs by the key, 8-bit digits. One read histograms all eight
+ *   digits; a pass whose digit is the same for every key is skipped. host_passes[3] = { passes run, passes skipped, 1 when the
+ *   sorted pairs are in dev_keys_alt / dev_vals_alt (an odd number of passes ran), else 0 }. 24 bytes per key in all.
+ * amwg_summary_rank_runs: run-length encoding of sorted keys: dev_run_id[n] = the run of each position, dev_run_keys[runs] (may
+ *   be NULL) the distinct keys, dev_run_counts[runs] their counts, or, when dev_weights is not NULL, the sum over the run of
+ *   dev_weights[dev_sorted_vals[i]] (the payloads index the weights; dev_sorted_vals may be NULL otherwise) and dev_weight_scan[n]
+ *   is the caller's scratch for their prefix sums (NULL without weights). *host_n_runs = runs.
+ * amwg_summary_rank_z: dev_run_z[i] = Phi^-1((r_i - 3/8) / (total + 1/4)) with the average 1-based rank
+ *   r_i = offset + (counts of the runs before i) + (count_i + 1) / 2. 0 <= offset, 1 <= total < 2^50. CUDA's normcdfinv.
+ *   dev_run_z must not overlap dev_run_counts (the counts are scanned in dev_run_z first).
+ * amwg_summary_rank_scatter: dev_out[((p / chains) * entries + entry) * chains + p % chains] = dev_run_z[dev_run_id[i]] with
+ *   p = dev_sorted_vals[i]: the z of each draw into a block [2h][entries][chains] (entries = 1, chains = n: dev_out[p]). */
+AMWG_API int amwg_summary_rank_keys(int device, const double* dev_samples, int64_t rows, int32_t entries, int64_t chains, int32_t entry,
+                                    const double* host_center, uint64_t* dev_keys, uint32_t* dev_vals);
+AMWG_API int amwg_summary_rank_sort(int device, uint64_t* dev_keys, uint32_t* dev_vals, int64_t n, uint64_t* dev_keys_alt,
+                                    uint32_t* dev_vals_alt, int32_t* host_passes);
+AMWG_API int amwg_summary_rank_runs(int device, const uint64_t* dev_sorted_keys, const uint32_t* dev_sorted_vals, const int64_t* dev_weights,
+                                    int64_t* dev_weight_scan, int64_t n, uint32_t* dev_run_id, uint64_t* dev_run_keys, int64_t* dev_run_counts,
+                                    int64_t* host_n_runs);
+AMWG_API int amwg_summary_rank_z(int device, const int64_t* dev_run_counts, int64_t n_runs, int64_t offset, int64_t total, double* dev_run_z);
+AMWG_API int amwg_summary_rank_scatter(int device, const uint32_t* dev_sorted_vals, const uint32_t* dev_run_id, int64_t n,
+                                       const double* dev_run_z, double* dev_out, int32_t entries, int64_t chains, int32_t entry);
+
 /* ---- run-time specialisation ----------------------------------------------------------------------------------------------
  * For models that run the statistics sweep (stat_prog) amwg_create generates CUDA source from the model's programs, compiles it
  * for sm_100a with NVRTC and steps with that kernel instead of the bytecode interpreter (csrc/amwg_jit.cuh; AMWG_JIT=0 in the

@@ -366,6 +366,50 @@ BINDING(summary_autocov)
     fail_from_library();
   return f64_array(env, out.data(), out.size());
 END_BINDING
+// summary_rank_keys(device, samples ptr, rows, entries, chains, entry, center (NaN: no fold), keys ptr, vals ptr)   amwg_summary_rank_keys
+BINDING(summary_rank_keys)
+  const double center = to_double(env, a.at(6));
+  if (amwg_summary_rank_keys((int)to_double(env, a.at(0)), (const double*)(uintptr_t)to_u64(env, a.at(1)), (int64_t)to_double(env, a.at(2)),
+                             (int32_t)to_double(env, a.at(3)), (int64_t)to_double(env, a.at(4)), (int32_t)to_double(env, a.at(5)),
+                             std::isnan(center) ? nullptr : &center, (uint64_t*)(uintptr_t)to_u64(env, a.at(7)), (uint32_t*)(uintptr_t)to_u64(env, a.at(8))) != 0)
+    fail_from_library();
+  return js_undefined(env);
+END_BINDING
+// summary_rank_sort(device, keys ptr, vals ptr, n, keys_alt ptr, vals_alt ptr) -> [passes run, skipped, in alt]   amwg_summary_rank_sort
+BINDING(summary_rank_sort)
+  int32_t passes[3] = {0, 0, 0};
+  if (amwg_summary_rank_sort((int)to_double(env, a.at(0)), (uint64_t*)(uintptr_t)to_u64(env, a.at(1)), (uint32_t*)(uintptr_t)to_u64(env, a.at(2)),
+                             (int64_t)to_double(env, a.at(3)), (uint64_t*)(uintptr_t)to_u64(env, a.at(4)), (uint32_t*)(uintptr_t)to_u64(env, a.at(5)), passes) != 0)
+    fail_from_library();
+  const double p[3] = {(double)passes[0], (double)passes[1], (double)passes[2]};
+  return f64_array(env, p, 3);
+END_BINDING
+// summary_rank_runs(device, sorted keys ptr, sorted vals ptr, weights ptr (0: none), weight scan ptr (0: none), n, run_id ptr,
+//                   run_keys ptr (0), run_counts ptr) -> runs                                   amwg_summary_rank_runs
+BINDING(summary_rank_runs)
+  int64_t runs = 0;
+  if (amwg_summary_rank_runs((int)to_double(env, a.at(0)), (const uint64_t*)(uintptr_t)to_u64(env, a.at(1)), (const uint32_t*)(uintptr_t)to_u64(env, a.at(2)),
+                             (const int64_t*)(uintptr_t)to_u64(env, a.at(3)), (int64_t*)(uintptr_t)to_u64(env, a.at(4)), (int64_t)to_double(env, a.at(5)),
+                             (uint32_t*)(uintptr_t)to_u64(env, a.at(6)), (uint64_t*)(uintptr_t)to_u64(env, a.at(7)), (int64_t*)(uintptr_t)to_u64(env, a.at(8)),
+                             &runs) != 0)
+    fail_from_library();
+  return js_number(env, (double)runs);
+END_BINDING
+// summary_rank_z(device, run_counts ptr, n_runs, offset, total, run_z ptr)      amwg_summary_rank_z
+BINDING(summary_rank_z)
+  if (amwg_summary_rank_z((int)to_double(env, a.at(0)), (const int64_t*)(uintptr_t)to_u64(env, a.at(1)), (int64_t)to_double(env, a.at(2)),
+                          (int64_t)to_double(env, a.at(3)), (int64_t)to_double(env, a.at(4)), (double*)(uintptr_t)to_u64(env, a.at(5))) != 0)
+    fail_from_library();
+  return js_undefined(env);
+END_BINDING
+// summary_rank_scatter(device, sorted vals ptr, run_id ptr, n, run_z ptr, out ptr, entries, chains, entry)   amwg_summary_rank_scatter
+BINDING(summary_rank_scatter)
+  if (amwg_summary_rank_scatter((int)to_double(env, a.at(0)), (const uint32_t*)(uintptr_t)to_u64(env, a.at(1)), (const uint32_t*)(uintptr_t)to_u64(env, a.at(2)),
+                                (int64_t)to_double(env, a.at(3)), (const double*)(uintptr_t)to_u64(env, a.at(4)), (double*)(uintptr_t)to_u64(env, a.at(5)),
+                                (int32_t)to_double(env, a.at(6)), (int64_t)to_double(env, a.at(7)), (int32_t)to_double(env, a.at(8))) != 0)
+    fail_from_library();
+  return js_undefined(env);
+END_BINDING
 // peak_fp64(device, reps) -> {tflops, ms}                                        amwg_peak_fp64
 BINDING(peak_fp64)
   double tf = 0.0, ms = 0.0;
@@ -404,7 +448,9 @@ NAPI_MODULE_INIT() {
       {"get_log_post", get_log_post}, {"set_adapting", set_adapting}, {"info", info}, {"kernel_launches", kernel_launches},
       {"last_sweep_kernel_ms", last_sweep_kernel_ms}, {"n_chains", n_chains}, {"last_error", last_error}, {"abi_version", abi_version},
       {"ld_eval", ld_eval}, {"primitive_eval", primitive_eval}, {"stream_uniforms", stream_uniforms}, {"device_log", device_log},
-      {"summary_moments", summary_moments}, {"summary_digit_hist", summary_digit_hist}, {"summary_autocov", summary_autocov}, {"peak_fp64", peak_fp64}, {"jit_status", jit_status},
+      {"summary_moments", summary_moments}, {"summary_digit_hist", summary_digit_hist}, {"summary_autocov", summary_autocov},
+      {"summary_rank_keys", summary_rank_keys}, {"summary_rank_sort", summary_rank_sort}, {"summary_rank_runs", summary_rank_runs},
+      {"summary_rank_z", summary_rank_z}, {"summary_rank_scatter", summary_rank_scatter}, {"peak_fp64", peak_fp64}, {"jit_status", jit_status},
       {"jit_compile_check", jit_compile_check}};
   for (const auto& e : table) {
     napi_value fn;
